@@ -507,6 +507,8 @@ def main():
                     "its own map replica and handle, registered concurrently on the one GPU (0/1 = skip)")
     ap.add_argument("--no-prefetch", action="store_true", help="e2e leg: upload each scan inside lsd_lio_scan instead of one scan ahead")
     ap.add_argument("--knn-batch", type=int, default=1 << 21, help="queries in the batched k-NN leg (N=1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path returned for its last step (state vector "
+                    "and covariance, float64) as DIR/<name>.npy, to compare two builds output for output")
     ap.add_argument("--mg-mode", default="replicas", choices=["replicas", "shard"],
                     help="N>1, what `value` / `e2e` report: 'replicas' = one map replica and one independent scan stream per GPU "
                          "(weak scaling, no collective); 'shard' = ONE scan stream, map tile-sharded across the GPUs, normal equations "
@@ -565,7 +567,8 @@ def main():
         return bool(getattr(lio, "_bench_sharded", False))
 
     def run_steps(lio, steps, scans, timed_from, prefetch=False):
-        """Returns (wall seconds of the timed part, per-step infos incl. host wall time per call, poses of ALL steps).
+        """Returns (wall seconds of the timed part, per-step infos incl. host wall time per call, poses of ALL steps, and the
+        state vector and covariance the last step returned).
         Bracketed by sync + barrier.  prefetch: the next scan is announced before the current one is registered (host
         scans: its H2D copy runs on the copy stream; any scan: its voxel grid is pipelined under the running scan)."""
         # Per-step inputs and outputs are laid out before the timed region (the priors are the workload's, not the path's);
@@ -605,7 +608,7 @@ def main():
             if len(infos) >= 2:
                 infos[-2]["gpu_ms"] = info["gpu_ms"]  # async insert: device time is reported one scan late
         infos[-1]["gpu_ms"] = last_ms
-        return wall, infos, poses
+        return wall, infos, poses, (states[-1], covs[-1])
 
     def run_mode(sharded):
         """The value leg (scans resident in HBM) and the e2e leg (pinned host scans, H2D inside) of one multi-GPU mode."""
@@ -626,7 +629,7 @@ def main():
         sampler = ClockSampler(local)
         sampler.start()
         time.sleep(0.3)
-        wall_a, infos_a, poses_a = run_steps(lio, steps_a, dev_scans, W, prefetch=True)
+        wall_a, infos_a, poses_a, last_a = run_steps(lio, steps_a, dev_scans, W, prefetch=True)
         clocks = sampler.stop()
         xchg = lio.shard_exchange_stats() if sharded else None     # over the timed steps of the value leg
         host_scans = [torch.from_numpy(stp[0]).pin_memory() for stp in steps_b]
@@ -634,7 +637,7 @@ def main():
         for hs in host_scans:  # first DMA from a freshly pinned buffer pays a one-off mapping cost: take it here
             scratch[:hs.shape[0]].copy_(hs, non_blocking=True)
         torch.cuda.synchronize()
-        wall_b, infos_b, _ = run_steps(lio, steps_b, host_scans, W, prefetch=not args.no_prefetch)
+        wall_b, infos_b, _, _ = run_steps(lio, steps_b, host_scans, W, prefetch=not args.no_prefetch)
         dev_ms = float(np.sum([i["gpu_ms"] for i in infos_a]))
         t = torch.tensor([wall_a, wall_b, dev_ms * 1e-3], dtype=torch.float64, device=dev)
         if dist is not None:
@@ -644,7 +647,7 @@ def main():
             assert i["pos_err"] < 0.1, f"LIO did not converge: {i}"
         streams = 1 if sharded else world
         return dict(xchg=xchg, lio=lio, st=st, build_s=build_s, steps_a=steps_a, steps_b=steps_b, dev_scans=dev_scans, host_scans=host_scans,
-                    infos_a=infos_a, infos_b=infos_b, poses_a=poses_a, clocks=clocks, wall_a=wall_a, wall_b=wall_b, dev_s=dev_s,
+                    infos_a=infos_a, infos_b=infos_b, poses_a=poses_a, last_a=last_a, clocks=clocks, wall_a=wall_a, wall_b=wall_b, dev_s=dev_s,
                     value=streams * K / wall_a, e2e=streams * K / wall_b, base=base)
 
     want_shard = world > 1 and args.mg_mode == "shard"
@@ -655,6 +658,11 @@ def main():
         other["lio"].close(); other["lio"] = None
     R = main_run
     lio, st, infos_a, infos_b = R["lio"], R["st"], R["infos_a"], R["infos_b"]
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        state, cov = R["last_a"]
+        np.save(os.path.join(args.dump_outputs, "state.npy"), np.asarray(state, np.float64))
+        np.save(os.path.join(args.dump_outputs, "cov.npy"), np.asarray(cov, np.float64))
     rho = st["points"] / max(st["cells"], 1)
 
     # H2D probe: what this box's PCIe path gives a 1.6 MB pinned copy (explains e2e - value)
@@ -699,7 +707,7 @@ def main():
         h.map.insert(m, 0)
         h.set_next_id(m.shape[0])
         h.set_reference_order(False)
-        wall_r, infos_r, poses_r = run_steps(h, R["steps_a"], R["dev_scans"], W, prefetch=True)
+        wall_r, infos_r, poses_r, _ = run_steps(h, R["steps_a"], R["dev_scans"], W, prefetch=True)
         ref_order_leg = {"value": K / wall_r, "unit": "scans/s", "ms_per_step": 1e3 * wall_r / K,
                          "device_ms_per_step": float(np.sum([i["gpu_ms"] for i in infos_r])) / K,
                          "vs_this_lines_value": (K / wall_r) / R["value"],

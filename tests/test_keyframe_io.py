@@ -1,11 +1,11 @@
 """Key-frame files (SURVEY.md section 8f row N3, the on-disk format): lsd_keyframe_save / lsd_keyframe_load and the pybind
 `dump_keyframe` against the reference's own KeyFrame::save / loadOdom / loadPcd compiled unmodified (oracle/ref_keyframe.cpp
--> oracle/_ref/libref_keyframe.so) and against the PCD reader the reference vendors (third_party/pypcd.py).  Host-only
-code: runs without a GPU."""
-import ctypes as C
+-> oracle/_ref/libref_keyframe.so) and against the PCD reader the reference vendors (third_party/pypcd.py), through what
+those wrote and read on the same seeded inputs (tests/golden/keyframe_ref.npz, tests/golden/make_golden_keyframe.py).
+Host-only code: runs without a GPU."""
+import hashlib
 import os
 import sys
-import types
 
 import numpy as np
 import pytest
@@ -13,18 +13,16 @@ import pytest
 import lsdreg
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_REF = os.path.join(os.path.dirname(_HERE), "oracle", "_ref", "libref_keyframe.so")
-needs_ref = pytest.mark.skipif(not os.path.exists(_REF), reason="oracle/_ref/libref_keyframe.so not built (needs /root/reference)")
+_GOLD = os.path.join(_HERE, "golden", "keyframe_ref.npz")
 
 
-def _ref():
-    L = C.CDLL(_REF)
-    f = np.ctypeslib.ndpointer(dtype=np.float32, flags="C_CONTIGUOUS")
-    d = np.ctypeslib.ndpointer(dtype=np.float64, flags="C_CONTIGUOUS")
-    L.ref_keyframe_save.argtypes = [C.c_char_p, C.c_uint64, C.c_long, f, C.c_int, d]
-    L.ref_keyframe_load.restype = C.c_int
-    L.ref_keyframe_load.argtypes = [C.c_char_p, C.POINTER(C.c_uint64), C.POINTER(C.c_long), d, f, C.c_int]
-    return L
+@pytest.fixture(scope="module")
+def gold():
+    return dict(np.load(_GOLD))
+
+
+def _sha(b) -> str:
+    return hashlib.sha256(b if isinstance(b, bytes) else np.ascontiguousarray(b).tobytes()).hexdigest()
 
 
 def _poses(rng):
@@ -45,25 +43,21 @@ def _cloud(rng, n):
     return p
 
 
-@needs_ref
-def test_files_equal_the_reference_writers_byte_for_byte(tmp_path):
-    L = _ref()
+def test_files_equal_the_reference_writers_byte_for_byte(tmp_path, gold):
     rng = np.random.default_rng(4)
     for k, T in enumerate(_poses(rng)):
         pts = _cloud(rng, 1000 + 37 * k)
         stamp, kid = 1_695_000_000_000_000 + 123_456 * k + 7, 40 + k
-        a, b = tmp_path / f"ours{k}", tmp_path / f"ref{k}"
-        a.mkdir(); b.mkdir()
+        a = tmp_path / f"ours{k}"
+        a.mkdir()
         lsdreg.keyframe_save(str(a), stamp, kid, pts, T)
-        L.ref_keyframe_save(os.fsencode(str(b)), stamp, kid, pts, pts.shape[0], np.ascontiguousarray(T, np.float64).reshape(-1))
-        assert (a / "data").read_bytes() == (b / "data").read_bytes(), (b / "data").read_text()
-        assert (a / "cloud.pcd").read_bytes() == (b / "cloud.pcd").read_bytes()
+        ref_data = gold[f"save{k}_data"].tobytes()
+        assert (a / "data").read_bytes() == ref_data, ref_data.decode()
+        assert _sha((a / "cloud.pcd").read_bytes()) == gold["save_pcd_sha256"][k]
         assert sorted(os.listdir(a)) == ["cloud.pcd", "data"]
 
 
-@needs_ref
-def test_each_side_loads_what_the_other_wrote(tmp_path):
-    L = _ref()
+def test_each_side_loads_what_the_other_wrote(tmp_path, gold):
     rng = np.random.default_rng(5)
     for k, T in enumerate(_poses(rng)[:4]):
         pts = _cloud(rng, 500 + k)
@@ -71,18 +65,18 @@ def test_each_side_loads_what_the_other_wrote(tmp_path):
         a, b = tmp_path / f"ours{k}", tmp_path / f"ref{k}"
         a.mkdir(); b.mkdir()
         lsdreg.keyframe_save(str(a), stamp, kid, pts, T)
-        L.ref_keyframe_save(os.fsencode(str(b)), stamp, kid, pts, pts.shape[0], np.ascontiguousarray(T, np.float64).reshape(-1))
+        (b / "data").write_bytes(gold[f"load{k}_data"].tobytes())
+        (b / "cloud.pcd").write_bytes(gold[f"load{k}_pcd"].tobytes())
         # ours <- reference's files
         s1, i1, T1, p1 = lsdreg.keyframe_load(str(b))
-        # reference <- our files
-        s2, i2 = C.c_uint64(), C.c_long()
-        T2 = np.zeros(16); p2 = np.zeros((pts.shape[0], 4), np.float32)
-        n2 = L.ref_keyframe_load(os.fsencode(str(a)), C.byref(s2), C.byref(i2), T2, p2, p2.shape[0])
+        # reference <- our files: the reference read its own files, and ours are the same bytes
+        assert (a / "data").read_bytes() == (b / "data").read_bytes() and (a / "cloud.pcd").read_bytes() == (b / "cloud.pcd").read_bytes()
+        s2, i2, T2, n2 = int(gold["load_stamp"][k]), int(gold["load_id"][k]), gold["load_T"][k], int(gold["load_n"][k])
         assert n2 == pts.shape[0] == p1.shape[0]
-        assert s1 == s2.value == stamp and i1 == i2.value == kid
-        np.testing.assert_array_equal(T1, T2.reshape(4, 4))
+        assert s1 == s2 == stamp and i1 == i2 == kid
+        np.testing.assert_array_equal(T1, T2)
         np.testing.assert_allclose(T1, T, rtol=1e-5, atol=1e-12)          # six significant digits survive the text file
-        np.testing.assert_array_equal(p1, p2)
+        assert _sha(np.ascontiguousarray(p1, np.float32)) == gold["load_pts_sha256"][k]      # p1 == what the reference loaded
         np.testing.assert_array_equal(p1[:, :3], pts[:, :3])
         np.testing.assert_allclose(p1[:, 3], pts[:, 3], rtol=3e-7)        # x 255 then / 255 in fp32
 
@@ -131,27 +125,13 @@ def test_pybind_dump_keyframe_writes_the_same_files(tmp_path):
         assert (a / f).read_bytes() == (b / f).read_bytes()
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/third_party/pypcd.py"), reason="reference tree absent")
-def test_cloud_pcd_is_read_by_the_reference_s_vendored_pcd_reader(tmp_path):
-    """third_party/pypcd.py is the PCD reader the reference ships for its Python tools; lzf (only needed for compressed
-    files) is not installed here and is stubbed, and numpy 2 dropped the binary mode of np.fromstring the reader was written
-    against, so that one call is routed to np.frombuffer."""
-    sys.modules.setdefault("lzf", types.ModuleType("lzf"))
-    sys.path.insert(0, "/root/reference/third_party")
-    try:
-        import pypcd
-    finally:
-        sys.path.remove("/root/reference/third_party")
+def test_cloud_pcd_is_read_by_the_reference_s_vendored_pcd_reader(tmp_path, gold):
+    """third_party/pypcd.py is the PCD reader the reference ships for its Python tools (run once on these inputs by
+    tests/golden/make_golden_keyframe.py): our cloud.pcd is the file it read, and what it read is the cloud."""
     rng = np.random.default_rng(8)
     pts = _cloud(rng, 777)
     d = tmp_path / "kf"; d.mkdir()
     lsdreg.keyframe_save(str(d), 5, 1, pts, np.eye(4))
-    real = np.fromstring
-    pypcd.np.fromstring = lambda buf, dtype=float, **kw: np.frombuffer(buf, dtype=dtype)
-    try:
-        pc = pypcd.PointCloud.from_path(str(d / "cloud.pcd"))
-    finally:
-        pypcd.np.fromstring = real
-    assert pc.points == 777 and list(pc.fields) == ["x", "y", "z", "intensity"]
-    np.testing.assert_array_equal(pc.pc_data["x"], pts[:, 0]); np.testing.assert_array_equal(pc.pc_data["z"], pts[:, 2])
-    np.testing.assert_array_equal(pc.pc_data["intensity"], pts[:, 3] * np.float32(255.0))
+    assert _sha((d / "cloud.pcd").read_bytes()) == gold["pypcd_pcd_sha256"]
+    assert int(gold["pypcd_points"]) == 777 and list(gold["pypcd_fields"]) == ["x", "y", "z", "intensity"]
+    assert list(gold["pypcd_sha256"]) == [_sha(pts[:, 0]), _sha(pts[:, 2]), _sha(pts[:, 3] * np.float32(255.0))]
